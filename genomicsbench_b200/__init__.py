@@ -95,6 +95,12 @@ class Engine:
         _check_arrays(pairs, seq_ref, seq_qer)
         self._rc(self._lib.bsw_extend(self._h, ptr(pairs), ptr(seq_ref), ptr(seq_qer), len(pairs), w))
 
+    def extend32(self, pairs: np.ndarray, seq_ref: np.ndarray, seq_qer: np.ndarray, w: int) -> None:
+        """bsw_extend32: ksw_extend2 in int32 for pairs outside extend()'s 16-bit domain (long-read flanks: lengths up
+        to 2^24 - 1, h0 + len2 * max score + end_bonus up to 2^30).  Results in place, like extend()."""
+        _check_arrays(pairs, seq_ref, seq_qer)
+        self._rc(self._lib.bsw_extend32(self._h, ptr(pairs), ptr(seq_ref), ptr(seq_qer), len(pairs), w))
+
     def extend_async(self, pairs: np.ndarray, seq_ref: np.ndarray, seq_qer: np.ndarray, w: int) -> int:
         """bsw_extend_async: queues the call, returns its ticket (the arrays must stay alive until wait())."""
         _check_arrays(pairs, seq_ref, seq_qer)

@@ -123,6 +123,7 @@ ABI = [
     ("bsw_last_error", C.c_char_p, [_P]),
     ("bsw_default_params", None, [C.POINTER(BswParams)]),
     ("bsw_extend", C.c_int, [_P, _P, _P, _P, C.c_int64, C.c_int32]),
+    ("bsw_extend32", C.c_int, [_P, _P, _P, _P, C.c_int64, C.c_int32]),
     ("bsw_extend_async", C.c_int, [_P, _P, _P, _P, C.c_int64, C.c_int32, C.POINTER(C.c_int64)]),
     ("bsw_wait", C.c_int, [_P, C.c_int64, C.POINTER(C.c_int64)]),
     ("bsw_async_stats", C.c_int, [_P, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),

@@ -23,6 +23,7 @@
 #include "bsw_kernels.cuh"
 #include "bsw_kernel16.cuh"
 #include "bsw_warp16.cuh"
+#include "bsw_long32.cuh"
 #include "bsw_prep.cuh"
 #include "bsw_global.cuh"
 #include "bsw_global2.cuh"
@@ -212,6 +213,7 @@ struct bsw_engine {
     bool cells_counted = false;           // the last run summed its effective cells itself (latency route): no device counters to collect
     void* clanes = nullptr;               // child engines of bsw_extend_chains' lanes (ChainLanes, bsw_chain.inl)
     void* aq = nullptr;                   // queue + worker of bsw_extend_async (AsyncQueue, bsw_async.inl)
+    void* x32bufs = nullptr;              // chunk buffers of bsw_extend32 (X32Bufs, bsw_extend32.inl)
     std::once_flag aq_once;
 };
 
@@ -1811,6 +1813,7 @@ bsw_engine* bsw_create(const bsw_params* params, int* err)
 static void bsw_global_release(bsw_engine* eng);      // bsw_global.inl
 static void bsw_chain_release(bsw_engine* eng);       // bsw_chain.inl
 static void bsw_async_release(bsw_engine* eng);       // bsw_async.inl
+static void bsw_extend32_release(bsw_engine* eng);    // bsw_extend32.inl
 
 void bsw_destroy(bsw_engine* eng)
 {
@@ -1818,6 +1821,7 @@ void bsw_destroy(bsw_engine* eng)
     bsw_async_release(eng);
     bsw_global_release(eng);
     bsw_chain_release(eng);
+    bsw_extend32_release(eng);
     for (DevCtx& c : eng->devs) {
         cudaSetDevice(c.dev);
         cudaDeviceSynchronize();
@@ -1934,15 +1938,14 @@ int bsw_extend_packed16(bsw_engine* eng, const bsw_packed_batch* batch, int32_t 
 // band-doubling retry (tools/bwa/bwamem.c:723-753, :770-800), batched: the pairs that neither
 // repeated their score nor stayed within 3/4 of the band are gathered and re-run with w << t
 // ------------------------------------------------------------------------------------------
-int bsw_extend_retry(bsw_engine* eng, SeqPair* pairs, const uint8_t* seq_ref, const uint8_t* seq_qer,
-                     int64_t n, int32_t w, int32_t max_try, const int32_t* prev_score, int32_t* band_used)
+typedef int (*ExtendFn)(bsw_engine*, SeqPair*, const uint8_t*, const uint8_t*, int64_t, int32_t);
+
+// the retry loop over one extension entry point (bsw_extend, or bsw_extend32 for bsw_extend_chains' long flanks);
+// arguments validated by the caller
+static int extend_retry_with(ExtendFn extend, bsw_engine* eng, SeqPair* pairs, const uint8_t* seq_ref, const uint8_t* seq_qer,
+                             int64_t n, int32_t w, int32_t max_try, const int32_t* prev_score, int32_t* band_used)
 {
-    if (!eng) return BSW_ERR_PARAM;
-    if (max_try < 1 || max_try > 8 || w < 0 || ((int64_t)w << (max_try - 1)) > 0x3fffffff) {
-        eng->err = "bsw_extend_retry: max_try must be in 1..8 and w << (max_try - 1) must fit";
-        return BSW_ERR_PARAM;
-    }
-    if (int rc = bsw_extend(eng, pairs, seq_ref, seq_qer, n, w)) return rc;
+    if (int rc = extend(eng, pairs, seq_ref, seq_qer, n, w)) return rc;
     bsw_stats total = eng->stats;
     std::vector<int64_t> active, next;
     std::vector<int32_t> prev;
@@ -1956,7 +1959,7 @@ int bsw_extend_retry(bsw_engine* eng, SeqPair* pairs, const uint8_t* seq_ref, co
         const int32_t wt = w << t;
         sub.resize(active.size());
         for (size_t k = 0; k < active.size(); ++k) sub[k] = pairs[active[k]];
-        if (int rc = bsw_extend(eng, sub.data(), seq_ref, seq_qer, (int64_t)sub.size(), wt)) return rc;
+        if (int rc = extend(eng, sub.data(), seq_ref, seq_qer, (int64_t)sub.size(), wt)) return rc;
         total.cells_effective += eng->stats.cells_effective; total.kernel_launches += eng->stats.kernel_launches;
         total.h2d_bytes += eng->stats.h2d_bytes; total.d2h_bytes += eng->stats.d2h_bytes;
         total.ms_kernel += eng->stats.ms_kernel; total.ms_pack += eng->stats.ms_pack; total.ms_scatter += eng->stats.ms_scatter;
@@ -1978,6 +1981,18 @@ int bsw_extend_retry(bsw_engine* eng, SeqPair* pairs, const uint8_t* seq_ref, co
     return BSW_OK;
 }
 
+int bsw_extend_retry(bsw_engine* eng, SeqPair* pairs, const uint8_t* seq_ref, const uint8_t* seq_qer,
+                     int64_t n, int32_t w, int32_t max_try, const int32_t* prev_score, int32_t* band_used)
+{
+    if (!eng) return BSW_ERR_PARAM;
+    if (max_try < 1 || max_try > 8 || w < 0 || ((int64_t)w << (max_try - 1)) > 0x3fffffff) {
+        eng->err = "bsw_extend_retry: max_try must be in 1..8 and w << (max_try - 1) must fit";
+        return BSW_ERR_PARAM;
+    }
+    return extend_retry_with(bsw_extend, eng, pairs, seq_ref, seq_qer, n, w, max_try, prev_score, band_used);
+}
+
+#include "bsw_extend32.inl"
 #include "bsw_chain.inl"
 #include "bsw_global.inl"
 #include "bsw_async.inl"

@@ -127,6 +127,16 @@ void        bsw_default_params(bsw_params* p);       /* bwa defaults: main_bande
 int bsw_extend(bsw_engine* eng, SeqPair* pairs, const uint8_t* seq_ref,
                const uint8_t* seq_qer, int64_t n_pairs, int32_t w);
 
+/* ---- long-read flanks --------------------------------------------------------
+ * replaces: ksw_extend2 (tools/bwa/ksw.c:380-479) with its int32 arithmetic, for pairs outside bsw_extend's
+ * 16-bit domain (long-read flanks).  Same SeqPair records, engine scoring, z-drop rule (zdrop_mode) and in-place
+ * result fields as bsw_extend; pads never written, pair.id never read.  Runs on the engine's first device.
+ * Domain (BSW_ERR_DOMAIN): 1 <= len1, len2 <= 2^24 - 1, h0 >= 0, h0 + len2 * mx + end_bonus <= 2^30
+ * (mx = largest score of the matrix, as in the band clamp).  Pairs inside bsw_extend's domain give bsw_extend's
+ * results. */
+int bsw_extend32(bsw_engine* eng, SeqPair* pairs, const uint8_t* seq_ref, const uint8_t* seq_qer,
+                 int64_t n_pairs, int32_t w);
+
 /* ---- the packed host format ---------------------------------------------------
  * The reference keeps file parsing outside its timed region (main_banded.cpp:262-270 loadPairs, :306 readTim) and
  * layout conversion inside it (the AoS->SoA transposes of bandedSWA.cpp:1266-1326).  A loader that emits THIS layout
