@@ -191,7 +191,14 @@ struct Job {
 };
 constexpr int BSW_RETRY_STAGED = -100;    // internal: the direct route met such a chunk; the call is run again on the staged route
 
+struct GlobalBufs;                        // bsw_global.inl
+struct X32Bufs;                           // bsw_extend32.inl
+struct ChainBufs;                         // bsw_chain.inl
+struct AsyncQueue;                        // bsw_async.inl
+
 } // namespace
+
+struct ChainLanes;                        // bsw_chain.inl
 
 struct bsw_engine {
     bsw_params p;
@@ -207,13 +214,12 @@ struct bsw_engine {
     int64_t n = 0;
     int32_t w = 0;
     std::vector<std::pair<int, int>> staged_chunks;   // (device, slot) per chunk, batch order
-    void* gbufs = nullptr;                // device buffers of bsw_global (GlobalBufs, bsw_global.inl)
-    bool global_attr_set = false, global2_attr_set = false;
-    void* cbufs = nullptr;                // page-locked staging of bsw_extend_chains (ChainBufs, bsw_chain.inl)
+    GlobalBufs* gbufs = nullptr;          // device buffers of bsw_global
+    ChainBufs* cbufs = nullptr;           // page-locked staging of bsw_extend_chains
     bool cells_counted = false;           // the last run summed its effective cells itself (latency route): no device counters to collect
-    void* clanes = nullptr;               // child engines of bsw_extend_chains' lanes (ChainLanes, bsw_chain.inl)
-    void* aq = nullptr;                   // queue + worker of bsw_extend_async (AsyncQueue, bsw_async.inl)
-    void* x32bufs = nullptr;              // chunk buffers of bsw_extend32 (X32Bufs, bsw_extend32.inl)
+    ChainLanes* clanes = nullptr;         // child engines of bsw_extend_chains' lanes
+    AsyncQueue* aq = nullptr;             // queue + worker of bsw_extend_async
+    X32Bufs* x32bufs = nullptr;           // chunk buffers of bsw_extend32
     std::once_flag aq_once;
 };
 
@@ -262,6 +268,68 @@ void release(Buf<T>& b)
     if (b.d) cudaFree(b.d);
     if (b.h) cudaFreeHost(b.h);
     b.d = nullptr; b.h = nullptr; b.cap = b.hcap = 0;
+}
+
+// One chunk in flight on the engine's first device (bsw_global, bsw_extend32): its stream, the events around its
+// kernels and the items of the call it holds.  The entry points add their own buffers on top.
+struct ChunkSlot {
+    cudaStream_t st{};
+    cudaEvent_t e0{}, e1{};
+    int64_t first = 0, m = 0;             // items [first, first + m) of the call
+    ChunkSlot() = default; ChunkSlot(const ChunkSlot&) = delete;     // owns its stream and events
+    ~ChunkSlot()
+    {
+        if (st) cudaStreamDestroy(st);
+        if (e0) cudaEventDestroy(e0);
+        if (e1) cudaEventDestroy(e1);
+    }
+    int open(bsw_engine* eng)             // stream and events, created on first use
+    {
+        if (!st) {
+            CUDA_TRY(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
+            CUDA_TRY(cudaEventCreate(&e0));
+            CUDA_TRY(cudaEventCreate(&e1));
+        }
+        return BSW_OK;
+    }
+    void add_kernel_ms(bsw_stats& S) const
+    {
+        float ms = 0;
+        if (cudaEventElapsedTime(&ms, e0, e1) == cudaSuccess) S.ms_kernel += (double)ms;
+    }
+};
+
+// Runs n items through two alternating slots: launch(k, first) prepares the chunk from item `first` on in slot k (and
+// sets its m) and enqueues its device work, finish(k) waits for slot k and moves its results out.  The host prepares
+// chunk j + 1 while the device runs chunk j; the slots drain in submission order.  An error returns only after the
+// device is synchronised, so that no copy still runs into a slot's or the caller's buffers.
+template <class SlotT, class LaunchFn, class FinishFn>
+int run_chunks(SlotT (&slot)[2], int64_t n, LaunchFn&& launch, FinishFn&& finish)
+{
+    bool pending[2] = {false, false};
+    int cur = 0;
+    for (int64_t next = 0; next < n || pending[0] || pending[1]; cur ^= 1) {
+        if (pending[cur]) {
+            if (int rc = finish(cur)) { cudaDeviceSynchronize(); return rc; }
+            pending[cur] = false;
+        }
+        if (next < n) {
+            if (int rc = launch(cur, next)) { cudaDeviceSynchronize(); return rc; }
+            pending[cur] = true;
+            next += slot[cur].m;
+        }
+    }
+    return BSW_OK;
+}
+
+// Frees an entry point's chunk slots (their destructors release their buffers) on the device they ran on.
+template <class BufsT>
+void free_chunk_bufs(bsw_engine* eng, BufsT*& b)
+{
+    if (!b) return;
+    if (!eng->devs.empty()) cudaSetDevice(eng->devs[0].dev);
+    delete b;
+    b = nullptr;
 }
 
 // Shared-memory words per thread (S).  S >= qlen + 8 (prefetched group, bsw_kernels.cuh), S / 4
