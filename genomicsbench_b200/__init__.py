@@ -140,6 +140,14 @@ class Engine:
         of pair i are cigar[cigar_off[i]:cigar_off[i + 1]] (len << 4 | op, op 0 M / 1 I / 2 D).
         out = (score int32[>= n], n_cigar int32[>= n], cigar uint32[cap], cigar_off int64[>= n + 1]): caller-owned
         result arrays, reused across calls like a C caller's; the returned arrays are then views of them."""
+        return self._global(self._lib.bsw_global, pairs, seq_ref, seq_qer, w, out)
+
+    def global_align32(self, pairs: np.ndarray, seq_ref: np.ndarray, seq_qer: np.ndarray, w, out=None) -> tuple:
+        """bsw_global32: global_align() for alignment regions of up to 2^24 - 1 bases (long-read regions), one warp
+        per alignment.  Same arguments, results and errors; inside global_align()'s domain the same results."""
+        return self._global(self._lib.bsw_global32, pairs, seq_ref, seq_qer, w, out)
+
+    def _global(self, fn, pairs, seq_ref, seq_qer, w, out) -> tuple:
         _check_arrays(pairs, seq_ref, seq_qer)
         n = len(pairs)
         wv = np.ascontiguousarray(np.broadcast_to(np.asarray(w, dtype=np.int32), (n,)))
@@ -148,14 +156,14 @@ class Engine:
             for a, dt, need in ((score, np.int32, n), (ncig, np.int32, n), (cigar, np.uint32, 1), (off, np.int64, n + 1)):
                 if a.dtype != dt or not a.flags.c_contiguous or len(a) < need:
                     raise ValueError("out = (score int32[n], n_cigar int32[n], cigar uint32[cap], cigar_off int64[n + 1]), contiguous")
-            self._rc(self._lib.bsw_global(self._h, ptr(pairs), ptr(seq_ref), ptr(seq_qer), n, ptr(wv), ptr(score),
-                                          ptr(ncig), ptr(cigar), len(cigar), ptr(off)))
+            self._rc(fn(self._h, ptr(pairs), ptr(seq_ref), ptr(seq_qer), n, ptr(wv), ptr(score), ptr(ncig), ptr(cigar),
+                        len(cigar), ptr(off)))
             return score[:n], cigar[:int(off[n])], off[:n + 1]
         score = np.zeros(max(n, 1), dtype=np.int32); ncig = np.zeros(max(n, 1), dtype=np.int32)
         cap = int((pairs["len1"].astype(np.int64) + pairs["len2"]).sum()) if n else 0
         cigar = np.zeros(max(cap, 1), dtype=np.uint32); off = np.zeros(n + 1, dtype=np.int64)
-        self._rc(self._lib.bsw_global(self._h, ptr(pairs), ptr(seq_ref), ptr(seq_qer), n, ptr(wv), ptr(score),
-                                      ptr(ncig), ptr(cigar), cap, ptr(off)))
+        self._rc(fn(self._h, ptr(pairs), ptr(seq_ref), ptr(seq_qer), n, ptr(wv), ptr(score), ptr(ncig), ptr(cigar), cap,
+                    ptr(off)))
         return score[:n], cigar[:int(off[n])].copy(), off
 
     def chain_window(self, w: int, l_pac: int, seeds: np.ndarray, l_query: int) -> tuple:

@@ -132,6 +132,7 @@ ABI = [
                                    C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     ("bsw_extend_chains", C.c_int, [_P, _P, C.c_int64, _P, _P, _P, _P, _P, _P]),
     ("bsw_global", C.c_int, [_P, _P, _P, _P, C.c_int64, _P, _P, _P, _P, C.c_int64, _P]),
+    ("bsw_global32", C.c_int, [_P, _P, _P, _P, C.c_int64, _P, _P, _P, _P, C.c_int64, _P]),
     ("bsw_host_alloc", _P, [C.c_size_t]),
     ("bsw_host_free", None, [_P]),
     ("bsw_host_register", C.c_int, [_P, C.c_size_t]),

@@ -28,6 +28,7 @@
 #include "bsw_global.cuh"
 #include "bsw_global2.cuh"
 #include "bsw_global_plan.h"
+#include "bsw_global32.cuh"
 #include <atomic>
 #include <cstdio>
 #include <cstring>
@@ -193,6 +194,7 @@ constexpr int BSW_RETRY_STAGED = -100;    // internal: the direct route met such
 
 struct GlobalBufs;                        // bsw_global.inl
 struct X32Bufs;                           // bsw_extend32.inl
+struct G32Bufs;                           // bsw_global32.inl
 struct ChainBufs;                         // bsw_chain.inl
 struct AsyncQueue;                        // bsw_async.inl
 
@@ -220,6 +222,7 @@ struct bsw_engine {
     ChainLanes* clanes = nullptr;         // child engines of bsw_extend_chains' lanes
     AsyncQueue* aq = nullptr;             // queue + worker of bsw_extend_async
     X32Bufs* x32bufs = nullptr;           // chunk buffers of bsw_extend32
+    G32Bufs* g32bufs = nullptr;           // chunk buffers of bsw_global32
     std::once_flag aq_once;
 };
 
@@ -270,7 +273,7 @@ void release(Buf<T>& b)
     b.d = nullptr; b.h = nullptr; b.cap = b.hcap = 0;
 }
 
-// One chunk in flight on the engine's first device (bsw_global, bsw_extend32): its stream, the events around its
+// One chunk in flight on the engine's first device (bsw_global, bsw_extend32, bsw_global32): its stream, the events around its
 // kernels and the items of the call it holds.  The entry points add their own buffers on top.
 struct ChunkSlot {
     cudaStream_t st{};
@@ -1882,6 +1885,7 @@ static void bsw_global_release(bsw_engine* eng);      // bsw_global.inl
 static void bsw_chain_release(bsw_engine* eng);       // bsw_chain.inl
 static void bsw_async_release(bsw_engine* eng);       // bsw_async.inl
 static void bsw_extend32_release(bsw_engine* eng);    // bsw_extend32.inl
+static void bsw_global32_release(bsw_engine* eng);    // bsw_global32.inl
 
 void bsw_destroy(bsw_engine* eng)
 {
@@ -1890,6 +1894,7 @@ void bsw_destroy(bsw_engine* eng)
     bsw_global_release(eng);
     bsw_chain_release(eng);
     bsw_extend32_release(eng);
+    bsw_global32_release(eng);
     for (DevCtx& c : eng->devs) {
         cudaSetDevice(c.dev);
         cudaDeviceSynchronize();
@@ -2063,6 +2068,7 @@ int bsw_extend_retry(bsw_engine* eng, SeqPair* pairs, const uint8_t* seq_ref, co
 #include "bsw_extend32.inl"
 #include "bsw_chain.inl"
 #include "bsw_global.inl"
+#include "bsw_global32.inl"
 #include "bsw_async.inl"
 
 // ------------------------------------------------------------------------------------------

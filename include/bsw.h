@@ -297,6 +297,21 @@ int bsw_global(bsw_engine* eng, const SeqPair* pairs, const uint8_t* seq_ref, co
                int64_t n_pairs, const int32_t* w, int32_t* score, int32_t* n_cigar, uint32_t* cigar,
                int64_t cigar_cap, int64_t* cigar_off);
 
+/* replaces: ksw_global2 (tools/bwa/ksw.c:502-606; push_cigar :489-500) with its int32 arithmetic, for alignment
+ * regions beyond bsw_global's 32767-base lengths (bwa_gen_cigar2 on long-read regions).  Same arguments, outputs,
+ * operation encoding, scoring and error codes as bsw_global; for any alignment inside bsw_global's domain the score
+ * and the operations are bsw_global's.  One warp per alignment; runs on the engine's first device.
+ * Domain (BSW_ERR_DOMAIN), checked for every alignment before any device work:
+ *   1 <= len1, len2 <= 2^24 - 1, offsets >= 0, |len1 - len2| <= w[i] (a band wider than max(len1, len2) is that band);
+ *   (len1 + len2 + 2) * c + o_del + o_ins <= 2^29, c = max(match, mismatch, |ambig|, e_del, e_ins): every real
+ *     H / E / F of the alignment lies in [-2^29, 2^29], far above the reference's -2^30 sentinel, and no sum
+ *     overflows (a path to any cell runs diagonally, then along one gap: at most max(len1, len2) + 2 steps of at most
+ *     c each and one gap open);
+ *   direction matrix len1 * 64 * ceil((min(len2, 2 w + 1) + 3) / 128) <= 2^31 bytes (4 bits per band cell). */
+int bsw_global32(bsw_engine* eng, const SeqPair* pairs, const uint8_t* seq_ref, const uint8_t* seq_qer,
+                 int64_t n_pairs, const int32_t* w, int32_t* score, int32_t* n_cigar, uint32_t* cigar,
+                 int64_t cigar_cap, int64_t* cigar_off);
+
 /* Pinned host memory.  bsw_extend takes any host pointers; when all three buffers (pairs,
  * seq_ref, seq_qer) are page-locked -- allocated here, or registered, or pinned by the caller's
  * own CUDA / torch allocator -- the engine DMAs them as they are and DMAs the records back with
