@@ -17,7 +17,7 @@ os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")
 
 import numpy as np
 
-from ._lib import (ABI, ALNREG_DTYPE, ALNREG_FIELDS, BSW_PACKED_MAX_QLEN, BSW_PAIR_RAW, BSW_ZDROP_SCALAR, BSW_ZDROP_VECTOR,
+from ._lib import (ABI, ALN_DTYPE, ALNREG_DTYPE, ALNREG_FIELDS, BSW_PACKED_MAX_QLEN, REG_IN_DTYPE, BSW_PAIR_RAW, BSW_ZDROP_SCALAR, BSW_ZDROP_VECTOR,
                    CHAIN_DTYPE, OUTSCORE_DTYPE, PAIR_DESC_DTYPE, RESULT_FIELDS, SCORE16_DTYPE, SEED_DTYPE, SEQPAIR_DTYPE,
                    BswChainOpt, BswGenConfig, BswPackedBatch, BswParams, BswStats, LIB_PATH, load_host_library,
                    load_library, ptr)
@@ -27,7 +27,8 @@ __all__ = [
     "gen_named_config", "gen_pairs", "bucket_order", "split_by_cost", "read_pairs_file",
     "write_pairs_file", "load_library", "NAMED_CONFIGS", "pinned_empty", "pinned_copy",
     "SEED_DTYPE", "CHAIN_DTYPE", "ALNREG_DTYPE", "ALNREG_FIELDS", "PackedBatch", "PAIR_DESC_DTYPE", "OUTSCORE_DTYPE",
-    "SCORE16_DTYPE", "BSW_PAIR_RAW", "BSW_PACKED_MAX_QLEN", "load_host_library",
+    "SCORE16_DTYPE", "BSW_PAIR_RAW", "BSW_PACKED_MAX_QLEN", "load_host_library", "REG_IN_DTYPE", "ALN_DTYPE",
+    "reg_inputs", "cigar_string", "reg2aln_capacity",
 ]
 
 NAMED_CONFIGS = {"small": 0, "short8": 1, "long16": 2, "large": 3, "sweep": 4}
@@ -196,6 +197,34 @@ class Engine:
                                              C.byref(opt), ptr(regs), ptr(count)))
         return regs[:len(seeds)], count[:len(chains)]
 
+    def reg2aln(self, regs_in: np.ndarray, query: np.ndarray, ref: np.ndarray, l_pac: int, w: int, out=None) -> tuple:
+        """mem_reg2aln's alignment part for a batch of regions (bsw_reg2aln; bwamem.c mem_reg2aln, bwa.c bwa_gen_cigar2):
+        band inference, the band-doubling loop, CIGAR with soft clips (ops "MIDSH": 3 = soft clip), NM and MD.
+        regs_in = REG_IN_DTYPE (reg_inputs builds it from extend_chains' output).  Returns (aln ALN_DTYPE[n],
+        cigar uint32[total], cigar_off int64[n + 1], md uint8[total], md_off int64[n + 1]); region i's operations are
+        cigar[cigar_off[i]:cigar_off[i + 1]], its MD md[md_off[i]:md_off[i + 1]] (ASCII, no NUL).
+        out = (aln ALN_DTYPE[>= n], cigar uint32[cap], cigar_off int64[>= n + 1], md uint8[cap], md_off int64[>= n + 1]):
+        caller-owned result arrays, reused across calls; the returned arrays are then views of them."""
+        regs_in = np.ascontiguousarray(regs_in, dtype=REG_IN_DTYPE)
+        if query.dtype != np.uint8 or ref.dtype != np.uint8 or not query.flags.c_contiguous or not ref.flags.c_contiguous:
+            raise ValueError("query / ref must be contiguous uint8 arrays (one base code per byte)")
+        n = len(regs_in)
+        if out is not None:
+            aln, cigar, coff, md, moff = out
+            for a, dt, need in ((aln, ALN_DTYPE, n), (cigar, np.uint32, 1), (coff, np.int64, n + 1), (md, np.uint8, 1),
+                                (moff, np.int64, n + 1)):
+                if a.dtype != dt or not a.flags.c_contiguous or len(a) < need:
+                    raise ValueError("out = (aln ALN_DTYPE[n], cigar uint32[cap], cigar_off int64[n + 1], md uint8[cap], "
+                                     "md_off int64[n + 1]), contiguous")
+        else:
+            ccap, mcap = reg2aln_capacity(regs_in)
+            aln = np.zeros(max(n, 1), dtype=ALN_DTYPE)
+            cigar, md = np.zeros(max(ccap, 1), dtype=np.uint32), np.zeros(max(mcap, 1), dtype=np.uint8)
+            coff, moff = np.zeros(n + 1, dtype=np.int64), np.zeros(n + 1, dtype=np.int64)
+        self._rc(self._lib.bsw_reg2aln(self._h, ptr(regs_in), n, ptr(query), ptr(ref), l_pac, w, ptr(aln), ptr(cigar),
+                                       len(cigar), ptr(coff), ptr(md), len(md), ptr(moff)))
+        return aln[:n], cigar[:int(coff[n])], coff[:n + 1], md[:int(moff[n])], moff[:n + 1]
+
     def extend_packed(self, batch: "PackedBatch", w: int, out: Optional[np.ndarray] = None, compact: bool = False) -> np.ndarray:
         """bsw_extend_packed / bsw_extend_packed16: a packed batch in, OUTSCORE_DTYPE (24 B) or SCORE16_DTYPE (16 B)
         records out, input order.  `out` = a caller-owned result array (page-locked for the DMA route)."""
@@ -280,6 +309,39 @@ class BandedPairWiseSW:
             if e is not None:
                 e.close()
         self._vec = self._scalar = None
+
+
+# ---------------------------------------------------------------------------------------
+# alignment records (bsw_reg2aln)
+# ---------------------------------------------------------------------------------------
+def reg_inputs(chains: np.ndarray, regs: np.ndarray, count: np.ndarray) -> np.ndarray:
+    """bsw_reg_in records for every region extend_chains() returned: the chain's read, and its reference bases
+    ref[chain.ref_off + rb - rmax0 ..] inside the chain's window (the same ref buffer extend_chains() read)."""
+    chains = np.asarray(chains, dtype=CHAIN_DTYPE)
+    idx = np.concatenate([np.arange(int(c["seed_first"]), int(c["seed_first"]) + int(k)) for c, k in zip(chains, count)]
+                         + [np.zeros(0, np.int64)]).astype(np.int64)
+    ch = np.repeat(np.arange(len(chains)), np.asarray(count, dtype=np.int64))
+    out = np.zeros(len(idx), dtype=REG_IN_DTYPE)
+    out["reg"] = regs[idx]
+    out["query_off"] = chains["query_off"][ch]
+    out["l_query"] = chains["l_query"][ch]
+    out["ref_off"] = chains["ref_off"][ch] + out["reg"]["rb"] - chains["rmax0"][ch]
+    return out
+
+
+def reg2aln_capacity(regs_in: np.ndarray) -> tuple:
+    """(cigar entries, MD bytes) that always suffice for these regions (include/bsw.h: (qe - qb) + (re - rb) + 2
+    operations and 4 (qe - qb) + (re - rb) + 1 MD bytes per mapped region)."""
+    r = regs_in["reg"]
+    mapped = (r["rb"] >= 0) & (r["re"] >= 0)
+    ql = np.where(mapped, r["qe"].astype(np.int64) - r["qb"], 0)
+    rl = np.where(mapped, r["re"] - r["rb"], 0)
+    return int((ql + rl + 2 * mapped).sum()), int((4 * ql + rl + mapped).sum())
+
+
+def cigar_string(ops) -> str:
+    """len << 4 | op operations -> CIGAR text with bwa's op letters "MIDSH" (3 = S)."""
+    return "".join(f"{int(c) >> 4}{'MIDSH'[int(c) & 0xf]}" for c in ops)
 
 
 # ---------------------------------------------------------------------------------------

@@ -65,6 +65,11 @@ CHAIN_DTYPE = np.dtype([("seed_first", "<i8"), ("n_seeds", "<i4"), ("l_query", "
 ALNREG_DTYPE = np.dtype([("rb", "<i8"), ("re", "<i8"), ("qb", "<i4"), ("qe", "<i4"), ("score", "<i4"), ("truesc", "<i4"),
                          ("w", "<i4"), ("seedcov", "<i4"), ("seedlen0", "<i4"), ("reserved", "<i4")])
 ALNREG_FIELDS = ("rb", "re", "qb", "qe", "score", "truesc", "w", "seedcov", "seedlen0")
+# include/bsw.h: bsw_reg_in (a region + where its read and reference bases are), bsw_aln (the alignment record)
+REG_IN_DTYPE = np.dtype([("reg", ALNREG_DTYPE), ("query_off", "<i8"), ("ref_off", "<i8"), ("l_query", "<i4"),
+                         ("reserved", "<i4")])
+ALN_DTYPE = np.dtype([("pos", "<i8"), ("is_rev", "<i4"), ("n_cigar", "<i4"), ("NM", "<i4"), ("gscore", "<i4"), ("w", "<i4"),
+                      ("reserved", "<i4")])
 
 
 class BswChainOpt(C.Structure):
@@ -133,6 +138,7 @@ ABI = [
     ("bsw_extend_chains", C.c_int, [_P, _P, C.c_int64, _P, _P, _P, _P, _P, _P]),
     ("bsw_global", C.c_int, [_P, _P, _P, _P, C.c_int64, _P, _P, _P, _P, C.c_int64, _P]),
     ("bsw_global32", C.c_int, [_P, _P, _P, _P, C.c_int64, _P, _P, _P, _P, C.c_int64, _P]),
+    ("bsw_reg2aln", C.c_int, [_P, _P, C.c_int64, _P, _P, C.c_int64, C.c_int32, _P, _P, C.c_int64, _P, _P, C.c_int64, _P]),
     ("bsw_host_alloc", _P, [C.c_size_t]),
     ("bsw_host_free", None, [_P]),
     ("bsw_host_register", C.c_int, [_P, C.c_size_t]),

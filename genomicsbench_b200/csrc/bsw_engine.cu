@@ -29,6 +29,7 @@
 #include "bsw_global2.cuh"
 #include "bsw_global_plan.h"
 #include "bsw_global32.cuh"
+#include "bsw_md.cuh"
 #include <atomic>
 #include <cstdio>
 #include <cstring>
@@ -195,6 +196,7 @@ constexpr int BSW_RETRY_STAGED = -100;    // internal: the direct route met such
 struct GlobalBufs;                        // bsw_global.inl
 struct X32Bufs;                           // bsw_extend32.inl
 struct G32Bufs;                           // bsw_global32.inl
+struct MdBufs;                            // bsw_reg2aln.inl
 struct ChainBufs;                         // bsw_chain.inl
 struct AsyncQueue;                        // bsw_async.inl
 
@@ -223,6 +225,7 @@ struct bsw_engine {
     AsyncQueue* aq = nullptr;             // queue + worker of bsw_extend_async
     X32Bufs* x32bufs = nullptr;           // chunk buffers of bsw_extend32
     G32Bufs* g32bufs = nullptr;           // chunk buffers of bsw_global32
+    MdBufs* mdbufs = nullptr;             // chunk buffers of bsw_reg2aln's finishing pass
     std::once_flag aq_once;
 };
 
@@ -1886,6 +1889,7 @@ static void bsw_chain_release(bsw_engine* eng);       // bsw_chain.inl
 static void bsw_async_release(bsw_engine* eng);       // bsw_async.inl
 static void bsw_extend32_release(bsw_engine* eng);    // bsw_extend32.inl
 static void bsw_global32_release(bsw_engine* eng);    // bsw_global32.inl
+static void bsw_reg2aln_release(bsw_engine* eng);     // bsw_reg2aln.inl
 
 void bsw_destroy(bsw_engine* eng)
 {
@@ -1895,6 +1899,7 @@ void bsw_destroy(bsw_engine* eng)
     bsw_chain_release(eng);
     bsw_extend32_release(eng);
     bsw_global32_release(eng);
+    bsw_reg2aln_release(eng);
     for (DevCtx& c : eng->devs) {
         cudaSetDevice(c.dev);
         cudaDeviceSynchronize();
@@ -2069,6 +2074,7 @@ int bsw_extend_retry(bsw_engine* eng, SeqPair* pairs, const uint8_t* seq_ref, co
 #include "bsw_chain.inl"
 #include "bsw_global.inl"
 #include "bsw_global32.inl"
+#include "bsw_reg2aln.inl"
 #include "bsw_async.inl"
 
 // ------------------------------------------------------------------------------------------

@@ -312,6 +312,58 @@ int bsw_global32(bsw_engine* eng, const SeqPair* pairs, const uint8_t* seq_ref, 
                  int64_t n_pairs, const int32_t* w, int32_t* score, int32_t* n_cigar, uint32_t* cigar,
                  int64_t cigar_cap, int64_t* cigar_off);
 
+/* ---- (f.5) alignment regions -> alignment records (CIGAR, NM, MD) ---------------------------
+ * replaces: the alignment part of mem_reg2aln (tools/bwa/bwamem.c, bwa 0.7.17) with infer_bw (bwamem.c) and
+ * bwa_gen_cigar2 (tools/bwa/bwa.c), bns_depos (bntseq.h), for every region of bsw_extend_chains' output:
+ *   w2 = max(infer_bw(qe-qb, re-rb, truesc, match, o_del, e_del), infer_bw(.., o_ins, e_ins)); if (w2 > w) w2 = min(w2, reg.w);
+ *   up to three tries:  w2 = min(w2, w << 2); bwa_gen_cigar2 with band w2;  stop if score == last score or
+ *                       w2 == w << 2;  else w2 <<= 1 and go on while score < truesc - match;
+ *   bwa_gen_cigar2:     rseq = ref bytes of [rb, re); for rb >= l_pac query segment and rseq are both reversed (indels
+ *                       come out leftmost in forward coordinates); l_query == re - rb and w2 == 0: one M run, score =
+ *                       sum of the column scores, no DP; else ksw_global2 (bsw_global / bsw_global32) with band
+ *                       max(min((max_gap + |rlen - l_query| + 1) >> 1, w2), |rlen - l_query| + 3), max_gap from
+ *                       (((l_query + 1) >> 1) * match - o) / e + 1 for both gap kinds, at least 1;  NM and MD over the
+ *                       (reversed) sequences, bases through "ACGTN" (rb < l_pac) or "TGCAN"; a D that is the first or
+ *                       the last operation is not in MD or NM; an I does not reset the match run;
+ *   then:               pos = rb < l_pac ? rb : 2 l_pac - 1 - (re - 1);  a leading D is dropped and moves pos, else a
+ *                       trailing D is dropped (only one end);  soft clips (op 3) of qb and l_query - qe bases, swapped
+ *                       when is_rev, are added at the ends.
+ * Operations are len << 4 | op in bwa's internal order "MIDSH": 0 = M, 1 = I, 2 = D, 3 = SOFT CLIP (not BAM's 4).
+ * regs[i].reg supplies rb re qb qe truesc w (the other fields are ignored); the read is
+ * query[query_off .. + l_query) (codes 0-4), the reference bases ref[ref_off .. + re - rb) as bns_get_seq(rb, re) returns
+ * them (for rb >= l_pac the reverse complement of the forward strand, i.e. D[rb, re) with D = G + revcomp(G)).  A region
+ * with rb < 0 or re < 0 gives the unmapped record: pos = -1, no operations, empty MD, no work.
+ * Outputs: out[i]; the operations of region i at cigar[cigar_off[i] .. cigar_off[i + 1]) (clips included); its MD at
+ * md[md_off[i] .. md_off[i + 1]) without a NUL.  cigar_off / md_off have n + 1 entries.  Capacities that always suffice,
+ * per region:  (qe - qb) + (re - rb) + 2 operations;  4 (qe - qb) + (re - rb) + 1 MD bytes (MD holds one number per
+ * mismatch and per inner D plus the last one, at most n_mm + n_D + 1 numbers, each of at most u + 1 digits for a run of
+ * u matches; the letters are n_mm mismatches and the deleted bases with one '^' per inner D; with
+ * sum u + n_mm <= qe - qb, n_mm <= qe - qb, n_D <= qe - qb (two D runs are separated by an operation that consumes query)
+ * and deleted bases <= re - rb the total is at most 4 (qe - qb) + (re - rb) + 1).  A buffer that cannot take the results
+ * gives BSW_ERR_PARAM (cigar: before any device work; md: after the chunks that fit are written).
+ * Domain (BSW_ERR_DOMAIN), checked for every region before any device work: 0 <= w <= 2^28; rb < re <= 2 l_pac, not
+ * bridging the strands (rb < l_pac < re); 0 <= qb < qe <= l_query; 1 <= l_query, re - rb <= 2^24 - 1; offsets >= 0;
+ * bsw_global32's value and direction-matrix bounds at the widest band the loop can reach.
+ * DP tries run through bsw_global (max(len1, len2) <= 32767) or bsw_global32 (longer); the finishing pass (NM, MD, the
+ * fast path's score) runs on the device.  Runs on the engine's first device.  Statistics: the sums over the call's DP
+ * calls and the finishing pass; ms_kernel includes both, ms_sort is the finishing pass's device time alone. */
+typedef struct bsw_reg_in {        /* one region to turn into an alignment record */
+    bsw_alnreg reg;                /* from bsw_extend_chains: rb re qb qe truesc w are read, the rest ignored */
+    int64_t query_off;             /* the read: query[query_off .. + l_query), codes 0-4 */
+    int64_t ref_off;               /* ref[ref_off .. + re - rb): the bases bns_get_seq(rb, re) returns */
+    int32_t l_query, reserved;
+} bsw_reg_in;
+typedef struct bsw_aln {           /* mem_aln_t's alignment fields */
+    int64_t pos;                   /* forward-strand 0-based leftmost position after the squeeze; -1 = unmapped */
+    int32_t is_rev, n_cigar, NM;
+    int32_t gscore;                /* global score of the last try (mem_aln_t.score is reg.score, the caller has it) */
+    int32_t w;                     /* band w2 of the last try */
+    int32_t reserved;
+} bsw_aln;
+int bsw_reg2aln(bsw_engine* eng, const bsw_reg_in* regs, int64_t n, const uint8_t* query, const uint8_t* ref,
+                int64_t l_pac, int32_t w, bsw_aln* out, uint32_t* cigar, int64_t cigar_cap, int64_t* cigar_off,
+                char* md, int64_t md_cap, int64_t* md_off);
+
 /* Pinned host memory.  bsw_extend takes any host pointers; when all three buffers (pairs,
  * seq_ref, seq_qer) are page-locked -- allocated here, or registered, or pinned by the caller's
  * own CUDA / torch allocator -- the engine DMAs them as they are and DMAs the records back with
