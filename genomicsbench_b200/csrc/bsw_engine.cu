@@ -399,11 +399,10 @@ struct WarpLease {
     WarpLease(const WarpLease&) = delete;
     WarpLease& operator=(const WarpLease&) = delete;
     ~WarpLease() { release(); }
-    bool acquire(const bsw_engine* eng, int cuda_dev, int64_t pairs, int e_ins, bool use16, int32_t limit_param)
+    bool acquire(const bsw_engine* eng, int cuda_dev, int64_t pairs, bool use16, int32_t limit_param)
     {
-        (void)eng;
         if (!use16 || limit_param < 0 || pairs <= 0 || cuda_dev < 0 || cuda_dev >= 64) return false;
-        if (7 * e_ins > 32767) return false;                    // the per-column decay of an entering F must fit 16 bits
+        if (!w16::scoring_ok(eng->kp)) return false;
         const int64_t limit = limit_param > 0 ? limit_param : WARP_MAX_PAIRS;
         std::atomic<int64_t>& g = g_warp_pairs[cuda_dev];
         int64_t cur = g.load(std::memory_order_relaxed);
@@ -423,7 +422,7 @@ struct WarpLease {
 // the static part of the rule, for a batch that stays resident (bsw_stage): no lease is held between its runs
 bool warp_fits(const bsw_engine* eng, int64_t n)
 {
-    if (!eng->use16 || eng->p.warp_max_pairs < 0 || n <= 0 || 7 * eng->kp.e_ins > 32767) return false;
+    if (!eng->use16 || eng->p.warp_max_pairs < 0 || n <= 0 || !w16::scoring_ok(eng->kp)) return false;
     return n <= (eng->p.warp_max_pairs > 0 ? eng->p.warp_max_pairs : WARP_MAX_PAIRS);
 }
 
@@ -1367,7 +1366,7 @@ int run_tiny(bsw_engine* eng, const Job& job, int dev_index, int64_t a0, int64_t
     Slot& s = *sp0;
     // Queries of at most 255 bases: the warp-per-pair register kernel (bsw_warp16.cuh) on 2-bit words packed by the host
     // pass.  A call with an N or a pair outside the 16-bit score domain keeps the byte route below.
-    if (qmax <= w16::MAX_QLEN && eng->use16 && eng->p.warp_max_pairs >= 0 && 7 * eng->kp.e_ins <= 32767) {
+    if (qmax <= w16::MAX_QLEN && eng->use16 && eng->p.warp_max_pairs >= 0 && w16::scoring_ok(eng->kp)) {
         if (int rc = set_kernel_attrs(eng, c)) return rc;
         const size_t off_desc = 64, off_q = off_desc + sizeof(int4) * (size_t)n;
         const size_t qwords = (size_t)(qtot / 16) + (size_t)n + 4, twords = (size_t)(rtot / 16) + (size_t)n + 4;
@@ -1397,7 +1396,7 @@ int run_tiny(bsw_engine* eng, const Job& job, int dev_index, int64_t a0, int64_t
             // a warp per pair while the device's budget of such pairs lasts (WarpLease), else the thread-per-pair kernel on
             // the same words: 0.4 ms per call instead of 0.14, but next to no load on a GPU whose issue rate is the bound
             WarpLease lease;
-            if (!lease.acquire(eng, c.dev, n, eng->kp.e_ins, eng->use16, eng->p.warp_max_pairs)) {
+            if (!lease.acquire(eng, c.dev, n, eng->use16, eng->p.warp_max_pairs)) {
                 const int qs = stride_for(qmax, true);
                 const int block = short16_block(qs, qs, false);
                 const int grid = (n + block - 1) / block;
@@ -1497,7 +1496,7 @@ int run_pipeline(bsw_engine* eng, const Job& job, int dev_lo, int ndev, int64_t 
     // long as it runs; a resident batch (its runs come later) and a batch dealt over several devices go by size alone
     WarpLease warp_lease;
     const bool warp_pairs = (keep || ndev != 1) ? warp_fits(eng, n)
-        : warp_lease.acquire(eng, eng->devs[(size_t)dev_lo].dev, n, eng->kp.e_ins, eng->use16, eng->p.warp_max_pairs);
+        : warp_lease.acquire(eng, eng->devs[(size_t)dev_lo].dev, n, eng->use16, eng->p.warp_max_pairs);
 
     // chunk boundaries: a small first chunk (the first DP starts after a short H2D), full-size
     // chunks, then -- where transfers or the host bound the batch -- a geometric ramp-down so that the

@@ -27,9 +27,17 @@
 //   column (the LAST one holding the maximum, bandedSWA.cpp:202-203) is resolved after the row
 //   from the h plane, and only when the row epilogue needs it.
 //
-// Domain of this kernel: (h0 + len2 * match) * (1 + match) <= 32767 (every intermediate fits 16
-// signed bits and the cap trick holds); the pack kernel routes everything else, and the pairs
-// that contain N, to the 32-bit byte kernel.
+// Domain of this kernel: (h0 + len2 * match) * (1 + match) <= 32767: every H, E, F and every
+// intermediate computed from them fits 16 signed bits and the cap trick holds.  The pack kernel
+// routes everything else, and the pairs that contain N, to the 32-bit byte kernel.
+// One computation may wrap, harmlessly: the row-maximum epilogue flags, with hs + (1 - m), the
+// halfwords of the block that holds the row maximum m plus one halfword on either side, and the
+// halfwords of columns from end on are not values of this row: they hold stale values, first-row
+// values or, never written, whatever shared memory held (a fill byte in the host emulation).  A
+// negative one v wraps whenever v + 1 - m < -32768 (for -32768 already at m = 2), and one above m
+// would be flagged; neither matters, because the flags of those columns, and of the two halfwords
+// outside the block, are masked off before the highest flag is taken.
+// tests/test_scoring_domain.py runs the emulation with several fill bytes and requires equal results.
 //
 // The row sweep is __host__ __device__: tests/k16_emu.cu runs it on the CPU with emulated DPX
 // instructions and an emulated shared-memory window, so the arithmetic is checked against the

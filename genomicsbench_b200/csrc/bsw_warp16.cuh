@@ -94,6 +94,10 @@ BSW_HD uint32_t mask_word(int lo, int hi, int k)
 
 BSW_HD int clamp08(int v) { v = v > 0 ? v : 0; return v < 8 ? v : 8; }
 
+// true when a scoring scheme may run on this kernel: the decay of an F entering a block at its last column, -7 e_ins
+// (dec3 in warp_sweep), must fit one signed halfword.  The engine's routes and the CPU emulation both ask this.
+BSW_HD bool scoring_ok(const KParams& P) { return 7 * P.e_ins <= 32767; }
+
 // a loop constant that stays in its register: ptxas otherwise re-derives it from the constant bank inside every row
 // (an LDC + two or three dependent instructions each; SASS of the first build)
 BSW_HD uint32_t pin(uint32_t x)

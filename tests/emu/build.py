@@ -9,12 +9,12 @@ HERE = Path(__file__).resolve().parent
 ROOT = HERE.parent.parent
 CSRC = ROOT / "genomicsbench_b200/csrc"
 DEPS = [CSRC / "bsw_kernel16.cuh", CSRC / "bsw_kernels.cuh", CSRC / "bsw_warp16.cuh", CSRC / "bsw_global2.cuh",
-        CSRC / "bsw_global_plan.h", CSRC / "bsw_global.cuh"]
+        CSRC / "bsw_global_plan.h", CSRC / "bsw_global.cuh", CSRC / "bsw_long32.cuh"]
 
 
 def build(force: bool = False, name: str = "k16") -> Path:
-    """name = "k16" (thread-per-pair sweep), "w16" (warp-per-pair register sweep, the lanes as coroutines) or "g2"
-    (bsw_global's second kernel with its chunk planner)."""
+    """name = "k16" (thread-per-pair sweep), "w16" (warp-per-pair register sweep, the lanes as coroutines), "l32" (the
+    int32 ring sweep of bsw_extend32, lanes as coroutines) or "g2" (bsw_global's second kernel with its chunk planner)."""
     so, src = HERE / f"lib{name}_emu.so", HERE / f"{name}_emu.cu"
     if not force and so.exists() and all(so.stat().st_mtime >= d.stat().st_mtime for d in DEPS + [src]):
         return so

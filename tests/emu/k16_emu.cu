@@ -35,8 +35,9 @@ extern "C" {
 // params: match, mismatch(+), o_del, e_del, o_ins, e_ins, zdrop, end_bonus, zmode
 // returns 0, or 1 when the pair is outside the packed kernel's domain; out6 = score qle tle gtle gscore max_off
 // circ != 0: circular rows of k16::circ_cols(w) columns (what the engine runs when the band is narrower than the query)
+// fill: the byte shared memory holds before the pair (the GPU leaves whatever was there; pads must not matter)
 int k16_emu_pair2(const int* prm, const uint8_t* q, int qlen, const uint8_t* t, int tlen, int h0, int w,
-                  int tid, int block, int circ, int* out6, long long* cells, long long* overflows)
+                  int tid, int block, int circ, int fill, int* out6, long long* cells, long long* overflows)
 {
     KParams P{};
     P.match = prm[0]; P.mismatch_neg = -prm[1]; P.ambig = -1;
@@ -48,7 +49,7 @@ int k16_emu_pair2(const int* prm, const uint8_t* q, int qlen, const uint8_t* t, 
     const int plane = stride_for(qlen);
     int qstride = plane, wcols = 0;
     if (circ && k16::circ_cols(w) + 4 < plane) { wcols = k16::circ_cols(w); qstride = wcols + 4; }
-    std::vector<uint8_t> smem(k16::smem_bytes(block, qstride, plane) + 64, 0xA5);   // garbage-filled: pads must not matter
+    std::vector<uint8_t> smem(k16::smem_bytes(block, qstride, plane) + 64, (uint8_t)fill);
     k16::emu_smem = smem.data();
     k16::emu_overflows = 0;
     uint32_t* tab = reinterpret_cast<uint32_t*>(smem.data());
@@ -80,12 +81,12 @@ int k16_emu_pair2(const int* prm, const uint8_t* q, int qlen, const uint8_t* t, 
 int k16_emu_pair(const int* prm, const uint8_t* q, int qlen, const uint8_t* t, int tlen, int h0, int w,
                  int tid, int block, int* out6, long long* cells, long long* overflows)
 {
-    return k16_emu_pair2(prm, q, qlen, t, tlen, h0, w, tid, block, 0, out6, cells, overflows);
+    return k16_emu_pair2(prm, q, qlen, t, tlen, h0, w, tid, block, 0, 0xA5, out6, cells, overflows);
 }
 
 // batch over SeqPair records (one base per byte, codes 0-3); skipped[i] = 1 for pairs outside the domain
 long long k16_emu_batch2(const int* prm, SeqPair* pairs, const uint8_t* ref, const uint8_t* qer, long long n, int w,
-                         int circ, uint8_t* skipped, long long* overflows)
+                         int circ, int fill, uint8_t* skipped, long long* overflows)
 {
     long long total = 0, ovf = 0;
 #pragma omp parallel for schedule(dynamic, 64) reduction(+ : total, ovf)
@@ -93,7 +94,7 @@ long long k16_emu_batch2(const int* prm, SeqPair* pairs, const uint8_t* ref, con
         SeqPair& sp = pairs[i];
         int out[6]; long long c = 0, o = 0;
         const int rc = k16_emu_pair2(prm, qer + sp.idq, sp.len2, ref + sp.idr, sp.len1, sp.h0, w,
-                                     (int)(i % 64), 64, circ, out, &c, &o);
+                                     (int)(i % 64), 64, circ, fill, out, &c, &o);
         if (skipped) skipped[i] = (uint8_t)rc;
         if (rc) continue;
         sp.score = out[0]; sp.qle = out[1]; sp.tle = out[2]; sp.gtle = out[3]; sp.gscore = out[4]; sp.max_off = out[5];
@@ -106,7 +107,7 @@ long long k16_emu_batch2(const int* prm, SeqPair* pairs, const uint8_t* ref, con
 long long k16_emu_batch(const int* prm, SeqPair* pairs, const uint8_t* ref, const uint8_t* qer, long long n, int w,
                         uint8_t* skipped, long long* overflows)
 {
-    return k16_emu_batch2(prm, pairs, ref, qer, n, w, 0, skipped, overflows);
+    return k16_emu_batch2(prm, pairs, ref, qer, n, w, 0, 0xA5, skipped, overflows);
 }
 
 } // extern "C"

@@ -80,7 +80,7 @@ struct WarpEmu {
     PairState sts[32];
     long long cells[32];
 
-    WarpEmu() : smem(w16::MASK_BYTES + WARPS * w16::SCORE_BYTES + 64, 0xA5), stacks(32 * STACK)    // garbage-filled: pads must not matter
+    explicit WarpEmu(int fill) : smem(w16::MASK_BYTES + WARPS * w16::SCORE_BYTES + 64, (uint8_t)fill), stacks(32 * STACK)
     {
         uint32_t* tab = reinterpret_cast<uint32_t*>(smem.data());
         for (int k = 0; k < w16::MASK_BYTES / 4; ++k) tab[k] = w16::mask_word((k >> 2) / 9, (k >> 2) % 9, k & 3);
@@ -132,21 +132,22 @@ extern "C" {
 
 // params: match, mismatch(+), o_del, e_del, o_ins, e_ins, zdrop, end_bonus, zmode.
 // batch over SeqPair records (one base per byte, codes 0-3); skipped[i] = 1 for pairs outside the kernel's domain
-// (16-bit scores, queries <= w16::MAX_QLEN).  Returns the effective cells, -1 when the lanes of a warp disagreed.
+// (w16::scoring_ok, 16-bit scores, queries <= w16::MAX_QLEN).  fill: the byte shared memory holds before the first pair
+// (pads must not matter).  Returns the effective cells, -1 when the lanes of a warp disagreed.
 long long w16_emu_batch(const int* prm, SeqPair* pairs, const uint8_t* ref, const uint8_t* qer, long long n, int w,
-                        uint8_t* skipped, long long* overflows)
+                        int fill, uint8_t* skipped, long long* overflows)
 {
     const KParams P = make_params(prm, w);
     const int nth = (int)std::max(1u, std::min(16u, std::thread::hardware_concurrency()));
     std::vector<long long> cells((size_t)nth, 0), ovf((size_t)nth, 0);
     std::vector<int> bad((size_t)nth, 0);
     auto worker = [&](int t) {
-        WarpEmu emu;
+        WarpEmu emu(fill);
         std::vector<uint32_t> qw, tw;
         k16::emu_overflows = 0;
         for (long long i = t; i < n; i += nth) {
             SeqPair& sp = pairs[i];
-            const bool ok = k16::eligible(P.match, sp.len2, sp.h0) && sp.len2 <= w16::MAX_QLEN;
+            const bool ok = w16::scoring_ok(P) && k16::eligible(P.match, sp.len2, sp.h0) && sp.len2 <= w16::MAX_QLEN;
             if (skipped) skipped[i] = ok ? 0 : 1;
             if (!ok) continue;
             pack2bit(qer + sp.idq, sp.len2, qw); pack2bit(ref + sp.idr, sp.len1, tw);

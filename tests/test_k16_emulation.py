@@ -17,19 +17,20 @@ def emu():
     lib = C.CDLL(str(build()))
     lib.k16_emu_batch2.restype = C.c_longlong
     lib.k16_emu_batch2.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.c_int,
-                                   C.c_void_p, C.c_void_p]
+                                   C.c_int, C.c_void_p, C.c_void_p]
     return lib
 
 
-def run_emu(lib, prm: dict, pairs, ref, qer, w, zmode=0, circ=0):
+def run_emu(lib, prm: dict, pairs, ref, qer, w, zmode=0, circ=0, fill=0xA5):
     """circ = 1: rows as circular buffers of the band's width wherever the band is narrower than the query
-    (what the engine launches then); circ = 0: rows that hold the whole query."""
+    (what the engine launches then); circ = 0: rows that hold the whole query.  fill = the byte shared memory holds
+    before a pair."""
     arr = np.array([prm["match"], prm["mismatch"], prm["o_del"], prm["e_del"], prm["o_ins"], prm["e_ins"],
                     prm["zdrop"], prm["end_bonus"], zmode], dtype=np.int32)
     skipped = np.zeros(len(pairs), dtype=np.uint8)
     ovf = C.c_longlong(0)
     cells = lib.k16_emu_batch2(arr.ctypes.data, pairs.ctypes.data, ref.ctypes.data, qer.ctypes.data, len(pairs), w,
-                               circ, skipped.ctypes.data, C.byref(ovf))
+                               circ, fill, skipped.ctypes.data, C.byref(ovf))
     return int(cells), skipped.astype(bool), int(ovf.value)
 
 

@@ -20,18 +20,19 @@ def emu():
     from emu.build import build
     lib = C.CDLL(str(build(name="w16")))
     lib.w16_emu_batch.restype = C.c_longlong
-    lib.w16_emu_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_int,
+    lib.w16_emu_batch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.c_int,
                                   C.c_void_p, C.c_void_p]
     return lib
 
 
-def run_emu(lib, prm: dict, pairs, ref, qer, w, zmode=0):
+def run_emu(lib, prm: dict, pairs, ref, qer, w, zmode=0, fill=0xA5):
+    """fill = the byte shared memory holds before the first pair."""
     arr = np.array([prm["match"], prm["mismatch"], prm["o_del"], prm["e_del"], prm["o_ins"], prm["e_ins"],
                     prm["zdrop"], prm["end_bonus"], zmode], dtype=np.int32)
     skipped = np.zeros(len(pairs), dtype=np.uint8)
     ovf = C.c_longlong(0)
     cells = lib.w16_emu_batch(arr.ctypes.data, pairs.ctypes.data, ref.ctypes.data, qer.ctypes.data, len(pairs), w,
-                              skipped.ctypes.data, C.byref(ovf))
+                              fill, skipped.ctypes.data, C.byref(ovf))
     assert cells >= 0
     return int(cells), skipped.astype(bool), int(ovf.value)
 
