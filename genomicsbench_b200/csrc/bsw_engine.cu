@@ -794,7 +794,8 @@ int staged_prepare(bsw_engine* eng, Slot& s, const SeqPair* pairs, const uint8_t
     const bool use16 = eng->use16;
     const int BLK = std::max(256, std::min(4096, n / (2 * eng->pool->size())));
     const int nblk = (n + BLK - 1) / BLK;
-    struct Sum { uint64_t qw = 0, rw = 0, rq = 0, rr = 0; };       // 2-bit words; RAW bytes of the long queries
+    struct Sum { uint64_t qw = 0, rw = 0, rq = 0, rr = 0, sq = 0, sr = 0; };    // 2-bit words; RAW bytes of the long
+                                                                                   // queries; bytes of the short pairs
     std::vector<Sum> sums((size_t)nblk + 1);
     std::vector<ChunkInfo> part((size_t)eng->pool->size());
     for (ChunkInfo& I : part) init_info(I);
@@ -812,6 +813,7 @@ int staged_prepare(bsw_engine* eng, Slot& s, const SeqPair* pairs, const uint8_t
             I.qmax_all = std::max(I.qmax_all, sp.len2);
             if (sp.len2 <= short_max) {
                 sm.qw += (uint64_t)((sp.len2 + 15) >> 4); sm.rw += (uint64_t)((sp.len1 + 15) >> 4);
+                sm.sq += (uint64_t)sp.len2; sm.sr += (uint64_t)sp.len1;
                 I.n_short++;
                 I.mn[0] = std::min(I.mn[0], sp.len2); I.mx[0] = std::max(I.mx[0], sp.len2);
                 I.mn[1] = std::min(I.mn[1], sp.h0);   I.mx[1] = std::max(I.mx[1], sp.h0);
@@ -835,13 +837,24 @@ int staged_prepare(bsw_engine* eng, Slot& s, const SeqPair* pairs, const uint8_t
     for (int b = 0; b < nblk; ++b) {
         sums[(size_t)b + 1].qw += sums[(size_t)b].qw; sums[(size_t)b + 1].rw += sums[(size_t)b].rw;
         sums[(size_t)b + 1].rq += sums[(size_t)b].rq; sums[(size_t)b + 1].rr += sums[(size_t)b].rr;
+        sums[(size_t)b + 1].sq += sums[(size_t)b].sq; sums[(size_t)b + 1].sr += sums[(size_t)b].sr;
+    }
+    // The descriptors hold 32-bit offsets, so a chunk's 2-bit words and its RAW bytes stay below 2^30 per side.  RAW
+    // bytes are the long queries' pairs plus the short pairs with N, which only pass 2 finds: every short pair counts as
+    // one here.  A chunk past either bound ends at its last block that keeps inside both (one block of at most 4096
+    // pairs always does: 4096 * 32767 < 2^30) and run_pipeline makes the rest its next chunk.  Pass 1 runs again on
+    // the shorter chunk so that its summary covers the chunk's pairs alone.
+    auto fits = [](const Sum& m) {
+        return m.qw <= 0x3fffffffull && m.rw <= 0x3fffffffull && m.rq + m.sq <= 0x3fffffffull && m.rr + m.sr <= 0x3fffffffull;
+    };
+    if (!fits(sums[(size_t)nblk])) {
+        int nb = nblk - 1;
+        while (nb > 1 && !fits(sums[(size_t)nb])) --nb;
+        s.n = nb * BLK;
+        return staged_prepare(eng, s, pairs, seq_ref, seq_qer);
     }
     const Sum tot = sums[(size_t)nblk];
     I.qbases = tot.qw * 16; I.tbases = tot.rw * 16;              // (they size the word arrays of device_prepare)
-    if (tot.qw > 0x3fffffffull || tot.rw > 0x3fffffffull || tot.rq > 0x3fffffffull || tot.rr > 0x3fffffffull) {
-        err_of(eng) = "chunk too large for 32-bit offsets";
-        return BSW_ERR_PARAM;
-    }
     if (int rc = ensure(eng, s.desc, (size_t)n, true)) return rc;
     if (int rc = ensure(eng, s.qraw, (size_t)tot.qw * 4 + 64, true)) return rc;
     if (int rc = ensure(eng, s.rraw, (size_t)tot.rw * 4 + 64, true)) return rc;
@@ -874,7 +887,6 @@ int staged_prepare(bsw_engine* eng, Slot& s, const SeqPair* pairs, const uint8_t
     // RAW side buffer: the long queries (offsets from pass 1), then the pairs with N
     uint64_t rq = tot.rq, rr = tot.rr;
     for (const std::vector<int>& v : with_n) for (int k : v) { rq += (uint64_t)P[k].len2; rr += (uint64_t)P[k].len1; }
-    if (rq > 0x3fffffffull || rr > 0x3fffffffull) { err_of(eng) = "chunk too large for 32-bit offsets"; return BSW_ERR_PARAM; }
     if (int rc = ensure(eng, s.rawq, (size_t)rq + 64, true)) return rc;
     if (int rc = ensure(eng, s.rawr, (size_t)rr + 64, true)) return rc;
     if (tot.rq > 0)
@@ -964,8 +976,16 @@ int staged_prepare_bytes(bsw_engine* eng, Slot& s, const SeqPair* pairs, const u
     }
     if (I.bad) return BSW_ERR_DOMAIN;
     for (int b = 0; b < nblk; ++b) { qsum[(size_t)b + 1] += qsum[(size_t)b]; rsum[(size_t)b + 1] += rsum[(size_t)b]; }
+    // 32-bit byte offsets: a chunk of more than 2^30 bytes on a side ends at its last block that fits (as in
+    // staged_prepare), and run_pipeline makes the rest its next chunk
+    auto fits = [&](int b) { return qsum[(size_t)b] <= 0x3fffffffull && rsum[(size_t)b] <= 0x3fffffffull; };
+    if (!fits(nblk)) {
+        int nb = nblk - 1;
+        while (nb > 1 && !fits(nb)) --nb;
+        s.n = nb * BLK;
+        return staged_prepare_bytes(eng, s, pairs, seq_ref, seq_qer);
+    }
     const uint64_t qtot = qsum[(size_t)nblk], rtot = rsum[(size_t)nblk];
-    if (qtot > 0x3fffffffull || rtot > 0x3fffffffull) { err_of(eng) = "chunk too large for 32-bit byte offsets"; return BSW_ERR_PARAM; }
     if (int rc = ensure(eng, s.desc, (size_t)n, true)) return rc;
     if (int rc = ensure(eng, s.qraw, (size_t)qtot + 64, true)) return rc;
     if (int rc = ensure(eng, s.rraw, (size_t)rtot + 64, true)) return rc;
@@ -1526,7 +1546,7 @@ int run_pipeline(bsw_engine* eng, const Job& job, int dev_lo, int ndev, int64_t 
         cut.push_back(cut.back() + sz);
         rem -= sz;
     }
-    const int64_t nchunks = (int64_t)cut.size() - 1;
+    int64_t nchunks = (int64_t)cut.size() - 1;          // (the staged route may end a chunk early: see split below)
     std::vector<ChunkRef> refs((size_t)nchunks);
     const double tl_host0 = now_ms();
     std::vector<std::string> tl_lines;
@@ -1620,6 +1640,20 @@ int run_pipeline(bsw_engine* eng, const Job& job, int dev_lo, int ndev, int64_t 
     const int lag = ndev;
     const int ahead = direct && !keep ? 3 * ndev : ndev;     // chunks opened (records + speculative sequence copy) ahead of k
     int64_t next_retire = 0;
+    // Staged route: the host pass ended chunk k early (its sequences would not fit 32-bit offsets).  The rest of its
+    // pairs become chunk k + 1, and the chunks opened after k move up one place: they are opened again at their new
+    // positions.  (On this route an open has done no work yet besides binding the chunk to its device and slot.)
+    auto split = [&](int64_t k, int n_fit) -> int {
+        cut.insert(cut.begin() + k + 1, cut[(size_t)k] + n_fit);
+        refs.emplace_back();
+        ++nchunks;
+        for (int64_t j = k + 1; j < std::min<int64_t>(k + ahead + 1, nchunks); ++j) {
+            if (!keep)
+                while (next_retire <= j - (int64_t)NSLOTS * ndev) if (int rc = retire(next_retire++)) return rc;
+            if (int rc = open(j)) return rc;
+        }
+        return BSW_OK;
+    };
     for (int64_t k = 0; k < std::min<int64_t>(ahead, nchunks); ++k) if (int rc = open(k)) return rc;
     for (int64_t k = 0; k < nchunks + lag; ++k) {
         if (k + ahead < nchunks) {
@@ -1628,11 +1662,17 @@ int run_pipeline(bsw_engine* eng, const Job& job, int dev_lo, int ndev, int64_t 
             if (int rc = open(k + ahead)) return rc;
         }
         if (k < nchunks) {
-            DevCtx& c = dev_of(k); Slot& s = slot_of(k);
+            DevCtx& c = dev_of(k);
             CUDA_TRY(cudaSetDevice(c.dev));
-            int rc = packed ? packed_info(eng, c, s)
-                   : direct ? direct_sequences(eng, s, pairs, seq_ref, seq_qer) : staged_prepare(eng, s, pairs, seq_ref, seq_qer);
+            int rc = packed ? packed_info(eng, c, slot_of(k))
+                   : direct ? direct_sequences(eng, slot_of(k), pairs, seq_ref, seq_qer)
+                   : staged_prepare(eng, slot_of(k), pairs, seq_ref, seq_qer);
             if (rc) { if (rc == BSW_ERR_DOMAIN) err_of(eng) = kDomainMsg; return rc; }
+            if (slot_of(k).n < cut[(size_t)k + 1] - cut[(size_t)k]) {
+                if ((rc = split(k, slot_of(k).n))) return rc;
+                CUDA_TRY(cudaSetDevice(c.dev));
+            }
+            Slot& s = slot_of(k);                          // (taken after split, whose opens may add slots)
             S.cells_nominal += (int64_t)s.info.nominal;
             if ((rc = device_prepare(eng, c, s))) return rc;
             if (g_timeline) s.host_t[1] = now_ms() - tl_host0;      // (after the wait for the summary + planning)
