@@ -357,11 +357,9 @@ inline int stride_for(int qmax, bool fine = false)
 // Block size of the packed kernel for a shared-memory class: a block's footprint (rows + query plane + 2 KB
 // score table + 1 KB the SM reserves) only fits the SM's 228 KB a whole number of times, and for some
 // classes 32-thread blocks leave less of it unused than 64-thread ones -- one more resident warp where
-// there are only four to seven.  BSW_SHORT_BLOCK=64 / 32 in the environment forces one size.
+// there are only four to seven.
 inline int short16_block(int qstride, int plane, bool circ)
 {
-    static const int forced = getenv("BSW_SHORT_BLOCK") ? atoi(getenv("BSW_SHORT_BLOCK")) : 0;
-    if (forced == 32 || forced == 64) return forced;
     const int sm_bytes = 228 * 1024;
     const int rb = circ ? 12 : 14;                    // register limit in blocks of 64: 71 registers, 77 with circular rows
     const int w64 = std::min((int)(sm_bytes / (k16::smem_bytes(64, qstride, plane) + 1024)), rb) * 2;
@@ -785,8 +783,7 @@ int staged_prepare_bytes(bsw_engine* eng, Slot& s, const SeqPair* pairs, const u
 // pair on the byte-reading warp-per-pair kernel) keeps the byte form of the pass.
 int staged_prepare(bsw_engine* eng, Slot& s, const SeqPair* pairs, const uint8_t* seq_ref, const uint8_t* seq_qer)
 {
-    static const bool bytes_only = getenv("BSW_STAGED_BYTES") && atoi(getenv("BSW_STAGED_BYTES")) != 0;   // A/B: round-1 form
-    if (s.tiny || bytes_only) return staged_prepare_bytes(eng, s, pairs, seq_ref, seq_qer);
+    if (s.tiny) return staged_prepare_bytes(eng, s, pairs, seq_ref, seq_qer);
     const double t0 = now_ms();
     const SeqPair* P = pairs + s.a;
     const int n = s.n;
@@ -1053,22 +1050,13 @@ int device_prepare(bsw_engine* eng, DevCtx& c, Slot& s)
         const int b_l2 = I.n_short ? bits_for((uint32_t)(I.mx[0] - I.mn[0])) : 0;        // <= 10: never shortened
         const int w_h0 = I.n_short ? bits_for((uint32_t)(I.mx[1] - I.mn[1])) : 0;
         const int w_l1 = I.n_short ? bits_for((uint32_t)(I.mx[2] - I.mn[2])) : 0;
-        // key = len2 | h0 | len1 cut to the bin table's BUCKET_BITS.  BSW_KEY_MODE (experiments): 0 = drop the low bits
-        // of the last field only (h0 exact, len1 coarse), 1 = len2 | len1 | h0 the same way, 2 = len2 | len1 | h0 with
-        // the dropped bits shared between both fields
-        // (measured, r02j_keymode.log: the orders differ by <= 2 %; 2 is never behind: short8 2.205 -> 2.167 ms, sweep w = 500 22.00 -> 21.58 ms)
-        static const int key_mode = getenv("BSW_KEY_MODE") ? atoi(getenv("BSW_KEY_MODE")) : 2;
+        // key = len2 | len1 | h0 cut to the bin table's BUCKET_BITS, the dropped low bits shared between len1 and h0
+        // (measured against dropping them from the last field only, r02j_keymode.log: never behind, short8 2.205 ->
+        // 2.167 ms, sweep w = 500 22.00 -> 21.58 ms)
         const int room = std::max(0, BUCKET_BITS - b_l2);
-        K.l1_first = key_mode != 0;
-        if (key_mode == 2) {
-            int k_l1 = std::min(w_l1, (room * 3 + 4) / 5), k_h0 = std::min(w_h0, room - k_l1);
-            k_l1 = std::min(w_l1, room - k_h0);
-            K.b_l1 = k_l1; K.b_h0 = k_h0;
-        } else if (key_mode == 1) {
-            K.b_l1 = std::min(w_l1, room); K.b_h0 = std::min(w_h0, room - K.b_l1);
-        } else {
-            K.b_h0 = std::min(w_h0, room); K.b_l1 = std::min(w_l1, room - K.b_h0);
-        }
+        int k_l1 = std::min(w_l1, (room * 3 + 4) / 5), k_h0 = std::min(w_h0, room - k_l1);
+        k_l1 = std::min(w_l1, room - k_h0);
+        K.b_l1 = k_l1; K.b_h0 = k_h0;
         K.s_h0 = w_h0 - K.b_h0; K.s_l1 = w_l1 - K.b_l1;
         const int total = b_l2 + K.b_h0 + K.b_l1;
         K.short_max = s.tiny ? 0 : eng->short_max;
@@ -1090,8 +1078,7 @@ int device_prepare(bsw_engine* eng, DevCtx& c, Slot& s)
         if (I.n_short > 0) {
             bsw_bucket_scan<<<ntiles, PREP_BLOCK, 0, s.st>>>(s.bins.d, nbins, totals, ticket);
             TL_MARK(2);
-            static const bool gather = getenv("BSW_PACKED_GATHER") && atoi(getenv("BSW_PACKED_GATHER")) != 0;   // A/B: re-lay the words in processing order
-            if (s.src2bit && !gather) {
+            if (s.src2bit) {
                 // packed route: the DP kernels read the 2-bit words where the host's DMA left them
                 bsw_bucket_scatter<true><<<grid_for(c, n, 2 * PREP_BLOCK), PREP_BLOCK, 0, s.st>>>(
                     s.desc.d, n, K, s.bins.d, totals, s.rank.d, s.perm.d, s.meta.d, s.nlist.d, s.d_info, s.q_lo, s.r_lo);
@@ -1102,21 +1089,15 @@ int device_prepare(bsw_engine* eng, DevCtx& c, Slot& s)
                 bsw_bucket_scatter<false><<<grid_for(c, n, 2 * PREP_BLOCK), PREP_BLOCK, 0, s.st>>>(s.desc.d, n, K, s.bins.d, totals, s.rank.d, s.perm.d);
                 TL_MARK(3);
                 // 2-bit packing in processing order
-                if (s.src2bit)
-                    bsw_pack_pairs<true><<<grid_for(c, I.n_short, PREP_BLOCK), PREP_BLOCK, 0, s.st>>>(
-                        s.desc.d, s.perm.d, I.n_short, s.q2src, s.r2src, s.meta.d, s.qpk.d, s.tpk.d, s.nlist.d, s.d_info, 0, 1,
-                        s.q_lo, s.r_lo);
-                else
-                    bsw_pack_pairs<false><<<grid_for(c, I.n_short, PREP_BLOCK), PREP_BLOCK, 0, s.st>>>(
-                        s.desc.d, s.perm.d, I.n_short, s.qbase, s.rbase, s.meta.d, s.qpk.d, s.tpk.d, s.nlist.d, s.d_info,
-                        s.use16 ? eng->p.match : 0, s.seq_on_device ? 1 : 0);
+                bsw_pack_pairs<<<grid_for(c, I.n_short, PREP_BLOCK), PREP_BLOCK, 0, s.st>>>(
+                    s.desc.d, s.perm.d, I.n_short, s.qbase, s.rbase, s.meta.d, s.qpk.d, s.tpk.d, s.nlist.d, s.d_info,
+                    s.use16 ? eng->p.match : 0, s.seq_on_device ? 1 : 0);
                 s.dp_q = s.qpk.d; s.dp_t = s.tpk.d;
                 stats_of(eng).kernel_launches += 3;
             }
             TL_MARK(4);
             // launch plan: the processing order ascends in len2, so the shared-memory classes are
             // prefix ranges of it, read off the len2 histogram
-            static const bool circ_ok = !(getenv("BSW_CIRC") && atoi(getenv("BSW_CIRC")) == 0);   // BSW_CIRC=0: rows always hold the whole query
             int pos = 0;
             for (int l = I.mn[0]; l <= std::min(I.mx[0], eng->short_max); ++l) {
                 const int cnt = (int)I.hist[l];
@@ -1124,7 +1105,7 @@ int device_prepare(bsw_engine* eng, DevCtx& c, Slot& s)
                 int qs = stride_for(l, s.use16);
                 int wc = 0;
                 const int plane = qs;
-                if (s.use16 && circ_ok && eng->kp.w <= 4096 && (k16::circ_cols(eng->kp.w) + 4) * 10 <= qs * 7) {
+                if (s.use16 && eng->kp.w <= 4096 && (k16::circ_cols(eng->kp.w) + 4) * 10 <= qs * 7) {
                     // the band is much narrower than the query: circular rows of the band's width (bsw_kernel16.cuh);
                     // every longer class then shares one row stride and merges into one launch.  Only where the
                     // rows shrink by 30 % or more: the wrap costs ~6 registers and a few instructions per block,
@@ -1476,9 +1457,9 @@ int run_tiny(bsw_engine* eng, const Job& job, int dev_index, int64_t a0, int64_t
 // Runs the chunks of the batch through the pipeline.  keep == true: stop before the DP launches
 // and keep every chunk resident in its own slot (bsw_stage).
 //
-// The call's pairs [a0, a0 + n) run on the devices [dev_lo, dev_lo + ndev) of the engine, chunks dealt round-robin
-// (run_sharded gives every device its own contiguous, cost-balanced range and its own host thread; bsw_stage deals
-// one range over all devices).
+// The call's pairs [a0, a0 + n) run on the devices [dev_lo, dev_lo + ndev) of the engine, chunks dealt round-robin.
+// Only bsw_stage (keep == true) deals over several devices; a call that runs (keep == false) has ndev == 1, since
+// run_sharded gives every device its own contiguous, cost-balanced range and its own host thread.
 int run_pipeline(bsw_engine* eng, const Job& job, int dev_lo, int ndev, int64_t a0, int64_t n, int64_t chunk_pairs, bool keep)
 {
     bsw_stats& S = stats_of(eng);
@@ -1487,9 +1468,8 @@ int run_pipeline(bsw_engine* eng, const Job& job, int dev_lo, int ndev, int64_t 
     const uint8_t* const seq_qer = job.seq_qer;
     const bool packed = job.pb != nullptr;
     const bool direct = packed || (!job.force_staged && is_pinned(pairs) && is_pinned(seq_ref) && is_pinned(seq_qer));
-    // direct route, way out: the records' device copy with the six fields filled in (72 B per pair, no host pass), or
-    // BSW_DIRECT_OUT=results: the 16-byte results + the staged route's host pass into the caller's records
-    static const bool out_records = !(getenv("BSW_DIRECT_OUT") && std::string(getenv("BSW_DIRECT_OUT")) == "results");
+    // direct route, way out: the records' device copy with the six fields filled in (72 B per pair, no host pass)
+    const bool out_records = direct && !packed;
     // PCIe-bound or compute-bound?  A sample of the records gives DP time (nominal cells at the
     // resident kernel rate) against transfer time (record + sequence bytes at PCIe rate) per pair.
     // PCIe-bound batches run partitioned: chunk streams on the service SMs, DP on the rest.
@@ -1513,9 +1493,9 @@ int run_pipeline(bsw_engine* eng, const Job& job, int dev_lo, int ndev, int64_t 
     S.partitioned = partitioned ? 1 : 0;
     const bool tiny = !keep && !packed && eng->p.tiny_batch > 0 && n <= eng->p.tiny_batch;
     // short pairs one per warp (bsw_warp16.cuh)?  A call on one device takes its pairs out of the device's budget for as
-    // long as it runs; a resident batch (its runs come later) and a batch dealt over several devices go by size alone
+    // long as it runs; a resident batch (its runs come later) goes by size alone
     WarpLease warp_lease;
-    const bool warp_pairs = (keep || ndev != 1) ? warp_fits(eng, n)
+    const bool warp_pairs = keep ? warp_fits(eng, n)
         : warp_lease.acquire(eng, eng->devs[(size_t)dev_lo].dev, n, eng->use16, eng->p.warp_max_pairs);
 
     // chunk boundaries: a small first chunk (the first DP starts after a short H2D), full-size
@@ -1525,18 +1505,15 @@ int run_pipeline(bsw_engine* eng, const Job& job, int dev_lo, int ndev, int64_t 
     // launch tails, better bucketing).
     // (pageable buffers: the host passes are the bottleneck and want large chunks for their thread pool)
     const bool small_chunks = pcie_bound && direct;
-    static const int64_t env_chunk = getenv("BSW_CHUNK") ? atoll(getenv("BSW_CHUNK")) : 0;          // experiments
-    static const int env_rampdown = getenv("BSW_RAMPDOWN") ? atoi(getenv("BSW_RAMPDOWN")) : -1;
-    const int64_t big = small_chunks ? CHUNK_PCIE : (env_chunk > 0 && !keep ? env_chunk : chunk_pairs);
+    const int64_t big = small_chunks ? CHUNK_PCIE : chunk_pairs;
     const int64_t tail_min = small_chunks ? CHUNK_MIN / 2 : CHUNK_MIN;    // the last chunk's latency is all tail
     // (a compute-bound batch on pinned buffers has all its data on the device long before the DP is done:
-    // small last chunks only add launches with few blocks -- scripts/chunk_probe.py: large mix 23.1 -> 21.9 ms)
-    const bool rampdown = env_rampdown >= 0 ? env_rampdown != 0 : (small_chunks || !direct);
+    // small last chunks only add launches with few blocks: large mix 23.1 -> 21.9 ms)
+    const bool rampdown = small_chunks || !direct;
     std::vector<int64_t> cut{a0};
-    static const int64_t env_first = getenv("BSW_FIRST_CHUNK") ? atoll(getenv("BSW_FIRST_CHUNK")) : 0;
     // (packed route, compute-bound: the whole batch arrives in a fraction of its DP time, and 64 k pairs -- half of what
     // the SMs hold at once -- start the DP 0.15 ms earlier than they cost in launch tails: 3.07 -> 2.93 ms per 1 M short pairs)
-    int64_t ramp = keep ? big : (env_first > 0 && !small_chunks ? env_first : (packed && !small_chunks ? 2 * CHUNK_MIN : CHUNK_MIN));
+    int64_t ramp = keep ? big : (packed && !small_chunks ? 2 * CHUNK_MIN : CHUNK_MIN);
     for (int64_t rem = n; rem > 0;) {
         int64_t sz;
         if (ramp < big && rem > 4 * ramp) { sz = ramp; ramp = small_chunks ? big : ramp * 2; }
@@ -1573,7 +1550,7 @@ int run_pipeline(bsw_engine* eng, const Job& job, int dev_lo, int ndev, int64_t 
         Slot& s = *sp;
         s.a = cut[(size_t)k]; s.n = (int)(cut[(size_t)k + 1] - cut[(size_t)k]);
         s.direct = direct;
-        s.out_records = direct && !packed && out_records;
+        s.out_records = out_records;
         s.packed = packed;
         s.src2bit = packed;                                   // (the staged route sets it in its host pass)
         s.tiny = tiny;
@@ -1608,7 +1585,7 @@ int run_pipeline(bsw_engine* eng, const Job& job, int dev_lo, int ndev, int64_t 
         unpack_chunk(eng, s, pairs);
         float ms = 0;
         if (cudaEventElapsedTime(&ms, s.ev_k0, s.ev_k1) == cudaSuccess) S.ms_kernel += (double)ms;
-        if (g_timeline && ndev == 1) {
+        if (g_timeline) {
             s.host_t[5] = now_ms() - tl_host0;
             char line[512];
             float t[7] = {};
@@ -1631,14 +1608,14 @@ int run_pipeline(bsw_engine* eng, const Job& job, int dev_lo, int ndev, int64_t 
         return BSW_OK;
     };
 
-    // Per iteration k: records (and the speculative sequence copy) of chunk k + 3 ndev go out (direct
+    // Per iteration k: records (and the speculative sequence copy) of chunk k + 3 go out (direct
     // route) so the copy engine never waits for the host; chunk k gets its prep kernels and DP launches; chunk
     // k - ndev drains (byte kernels, results out).  Chunks retire (results on the host; staged route:
     // second host pass) as soon as their D2H has completed, without blocking -- the host only waits
     // for a chunk when the slot it occupies is needed again, NSLOTS chunks later, so that a DP that
     // runs long never keeps the host from feeding the copy engine.
     const int lag = ndev;
-    const int ahead = direct && !keep ? 3 * ndev : ndev;     // chunks opened (records + speculative sequence copy) ahead of k
+    const int ahead = direct && !keep ? 3 : ndev;            // chunks opened (records + speculative sequence copy) ahead of k
     int64_t next_retire = 0;
     // Staged route: the host pass ended chunk k early (its sequences would not fit 32-bit offsets).  The rest of its
     // pairs become chunk k + 1, and the chunks opened after k move up one place: they are opened again at their new
@@ -1731,24 +1708,19 @@ inline double pair_cost(int len1, int len2, int w)
 // (sum of len1 * min(len2, 2w + 1), read off a sample of the records), each range runs through the chunk pipeline of
 // its own device on its own host thread, and every chunk's results land at its pairs' input positions.  Contiguous
 // ranges keep the host side free of any gather / scatter pass and every copy a plain DMA; the length bucketing
-// happens per chunk on the device.  BSW_MULTI=deal in the environment restores the single-thread round-robin
-// dealing of chunks over the devices (kept for A/B measurements, scripts/multi_probe.py).
+// happens per chunk on the device.
 int run_sharded(bsw_engine* eng, const Job& job, int64_t n, int64_t chunk_pairs)
 {
     const int ndev = (int)eng->devs.size();
     eng->cells_counted = false;
     if (!job.pb && eng->p.tiny_batch > 0 && n <= eng->p.tiny_batch) {
-        static const bool fused = !(getenv("BSW_TINY_FUSED") && atoi(getenv("BSW_TINY_FUSED")) == 0);     // A/B: 0 = the chunk pipeline's latency route
-        if (fused) {
-            const int rc = run_tiny(eng, job, 0, 0, n);
-            if (rc != 1) { eng->stats.shards = 1; eng->cells_counted = true; return rc; }      // (the results carried their cell counts)
-        }
+        const int rc = run_tiny(eng, job, 0, 0, n);
+        if (rc != 1) { eng->stats.shards = 1; eng->cells_counted = true; return rc; }      // (the results carried their cell counts)
     }
     if (int rc = zero_cells(eng)) return rc;
-    static const bool deal = getenv("BSW_MULTI") && std::string(getenv("BSW_MULTI")) == "deal";
     eng->stats.shards = 1;
-    if (ndev == 1 || deal) return run_pipeline(eng, job, 0, ndev, 0, n, chunk_pairs, false);
-    if (n < (int64_t)ndev * CHUNK_MIN) return run_pipeline(eng, job, 0, 1, 0, n, chunk_pairs, false);   // too small to split
+    if (ndev == 1 || n < (int64_t)ndev * CHUNK_MIN)                         // one device, or too small to split
+        return run_pipeline(eng, job, 0, 1, 0, n, chunk_pairs, false);
     eng->stats.shards = ndev;
     // cost curve from a sample (every step-th pair), cut at equal cost
     const int64_t step = std::max<int64_t>(1, n / 8192);
@@ -2131,13 +2103,12 @@ int bsw_stage(bsw_engine* eng, const SeqPair* pairs, const uint8_t* seq_ref, con
         if (int rc = zero_cells(eng)) return rc;
         Job job;
         job.pairs = const_cast<SeqPair*>(pairs); job.seq_ref = seq_ref; job.seq_qer = seq_qer;
-        static const int64_t env_stage = getenv("BSW_STAGE_CHUNK") ? atoll(getenv("BSW_STAGE_CHUNK")) : 0;     // experiments
-        int rc = run_pipeline(eng, job, 0, (int)eng->devs.size(), 0, n, env_stage > 0 ? env_stage : CHUNK_STAGE, true);
+        int rc = run_pipeline(eng, job, 0, (int)eng->devs.size(), 0, n, CHUNK_STAGE, true);
         if (rc == BSW_RETRY_STAGED) {
             quiesce(eng);
             job.force_staged = true;
             eng->stats.cells_nominal = 0; eng->stats.h2d_bytes = 0; eng->stats.kernel_launches = 0;
-            rc = run_pipeline(eng, job, 0, (int)eng->devs.size(), 0, n, env_stage > 0 ? env_stage : CHUNK_STAGE, true);
+            rc = run_pipeline(eng, job, 0, (int)eng->devs.size(), 0, n, CHUNK_STAGE, true);
         }
         if (rc != BSW_OK) { quiesce(eng); return rc; }
     }

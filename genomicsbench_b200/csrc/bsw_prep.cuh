@@ -279,16 +279,13 @@ __device__ __forceinline__ uint32_t bsw_pack16(const uint8_t* src, int nb, int r
 // found by binary search), so loads stay coalesced for short and long sequences alike.  The output
 // range is reserved once per block tile (two atomics on the chunk's cursors per block).
 // meta[s] (processing order) gets word offsets; desc[i] (input order) keeps byte offsets.
-// SRC2BIT (packed route): the sources are the chunk's 2-bit words as the host packed them (qraw / rraw point at the
-// chunk's first word, word_lo = that word's offset in the batch); words are copied instead of packed, and RAW pairs
-// (bsw_pair_desc.flags, desc.w >> 16) contribute no words and are listed for the byte kernel like pairs with N.
-template <bool SRC2BIT>
+// The sources are one byte per base (the staged and direct routes); the packed route's 2-bit words are read in
+// place by the DP kernels and never pass through here.
 __global__ void __launch_bounds__(PREP_BLOCK)
 bsw_pack_pairs(const int4* __restrict__ desc, const uint32_t* __restrict__ perm, int n_sorted,
                const uint8_t* __restrict__ qraw, const uint8_t* __restrict__ rraw, int4* __restrict__ meta,
                uint32_t* __restrict__ qpk, uint32_t* __restrict__ tpk,
-               uint32_t* __restrict__ nlist, ChunkInfo* __restrict__ info, int packed16_match, int overread,
-               unsigned int q_word_lo = 0, unsigned int r_word_lo = 0)
+               uint32_t* __restrict__ nlist, ChunkInfo* __restrict__ info, int packed16_match, int overread)
 {
     constexpr int NW = PREP_BLOCK / 32;
     __shared__ uint32_t s_pre[NW][2][33];
@@ -307,9 +304,8 @@ bsw_pack_pairs(const int4* __restrict__ desc, const uint32_t* __restrict__ perm,
             len2 = d.z & 0xffff; len1 = (d.z >> 16) & 0xffff;
         }
         s_desc[wib][lane] = d;
-        const bool is_raw = SRC2BIT && ((d.w >> 16) & BSW_PAIR_RAW) != 0;
-        const uint32_t nq = is_raw ? 0u : (uint32_t)(len2 + 15) >> 4;
-        const uint32_t nt = is_raw ? 0u : (uint32_t)(len1 + 15) >> 4;
+        const uint32_t nq = (uint32_t)(len2 + 15) >> 4;
+        const uint32_t nt = (uint32_t)(len1 + 15) >> 4;
         uint32_t pq = nq, pt = nt;                  // inclusive warp scans
 #pragma unroll
         for (int o = 1; o < 32; o <<= 1) {
@@ -344,29 +340,21 @@ bsw_pack_pairs(const int4* __restrict__ desc, const uint32_t* __restrict__ perm,
                     if (pre[lo + step] <= wv) lo += step;
                 const int4 dd = s_desc[wib][lo];
                 const uint32_t wi = wv - pre[lo];
-                if (SRC2BIT) {
-                    const uint32_t* srcw = kind ? reinterpret_cast<const uint32_t*>(rraw) + ((uint32_t)dd.y - r_word_lo)
-                                                : reinterpret_cast<const uint32_t*>(qraw) + ((uint32_t)dd.x - q_word_lo);
-                    (kind ? tpk + bt : qpk + bq)[wv] = __ldg(srcw + wi);
-                } else {
-                    const int len = kind ? (dd.z >> 16) & 0xffff : dd.z & 0xffff;
-                    const uint8_t* src = (kind ? rraw + dd.y : qraw + dd.x) + 16 * (int)wi;
-                    uint32_t bad = 0;
-                    const int room = len - 16 * (int)wi;
-                    const uint32_t word = bsw_pack16(src, min(16, room), room, bad, overread != 0);
-                    (kind ? tpk + bt : qpk + bq)[wv] = word;
-                    if (bad) atomicOr(&s_bad[wib][lo], 1u);
-                }
+                const int len = kind ? (dd.z >> 16) & 0xffff : dd.z & 0xffff;
+                const uint8_t* src = (kind ? rraw + dd.y : qraw + dd.x) + 16 * (int)wi;
+                uint32_t bad = 0;
+                const int room = len - 16 * (int)wi;
+                const uint32_t word = bsw_pack16(src, min(16, room), room, bad, overread != 0);
+                (kind ? tpk + bt : qpk + bq)[wv] = word;
+                if (bad) atomicOr(&s_bad[wib][lo], 1u);
             }
         }
         __syncwarp();
         if (s < n_sorted) {
             // pairs for the 32-bit byte kernel: those that contain N and, when the packed 16-bit kernel
             // runs the rest (packed16_match = its match score), those outside its score domain
-            // (packed route: a chunk with 2-bit pairs outside that domain runs the 32-bit kernel as a whole)
-            const bool has_n = SRC2BIT ? is_raw
-                                       : s_bad[wib][lane] != 0 ||
-                                         (packed16_match > 0 && !k16::eligible(packed16_match, len2, d.w & 0xffff));
+            const bool has_n = s_bad[wib][lane] != 0 ||
+                               (packed16_match > 0 && !k16::eligible(packed16_match, len2, d.w & 0xffff));
             meta[s] = make_int4((int)(bq + pq - nq), (int)(bt + pt - nt), d.z, (d.w & 0xffff) | (has_n ? BSW_META_NFLAG : 0));
             if (has_n) { nlist[atomicAdd(&info->n_nlist, 1u)] = (uint32_t)pi; atomicMax(&info->qmax_n, len2); }
         }
@@ -374,12 +362,11 @@ bsw_pack_pairs(const int4* __restrict__ desc, const uint32_t* __restrict__ perm,
     }
 }
 
-// ---- bucketing: counting sort by the compressed key (len2 | h0 | len1) >> drop --------------
+// ---- bucketing: counting sort by the compressed key (len2 | len1 | h0) >> drop --------------
 struct BucketKey {
     int mn2, mnh, mn1;        // minima of len2, h0, len1
     int b_h0, b_l1;           // bit widths of the h0 and len1 fields (after their shifts)
     int s_h0, s_l1;           // low bits dropped from h0 - mnh / len1 - mn1 so that the key fits the bin table
-    int l1_first;             // field order below len2: 1 = len1 then h0, 0 = h0 then len1
     int short_max;
 };
 
@@ -387,8 +374,7 @@ __device__ __forceinline__ uint32_t bsw_bucket_of(const BucketKey& K, const int4
 {
     const uint32_t len2 = d.z & 0xffff, len1 = (d.z >> 16) & 0xffff, h0 = d.w & 0xffff;
     const uint32_t a = (h0 - K.mnh) >> K.s_h0, b = (len1 - K.mn1) >> K.s_l1;
-    const uint32_t low = K.l1_first ? (b << K.b_h0) | a : (a << K.b_l1) | b;
-    return ((len2 - K.mn2) << (K.b_h0 + K.b_l1)) | low;
+    return ((len2 - K.mn2) << (K.b_h0 + K.b_l1)) | (b << K.b_h0) | a;
 }
 
 // rank[i] = arrival order of pair i inside its bin; bins[] accumulates the bin sizes; pairs whose

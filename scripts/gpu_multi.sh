@@ -14,20 +14,15 @@ TR="python -m torch.distributed.run --nnodes=1 --nproc-per-node $N --master-addr
 timeout 300 $TR --master-port 29610 scripts/fabric_probe.py > $OUT/${TAG}_fabric_n$N.json 2> $OUT/${TAG}_fabric_n$N.err; tail -25 $OUT/${TAG}_fabric_n$N.json
 timeout 600 python -m pytest tests -m gpu -x -q -k "devices or partitioner" > $OUT/${TAG}_pytest_multi_n$N.log 2>&1; tail -3 $OUT/${TAG}_pytest_multi_n$N.log
 timeout 400 python scripts/multi_probe.py --max-devices $N > $OUT/${TAG}_multi_probe_shard_n$N.log 2>&1; tail -1 $OUT/${TAG}_multi_probe_shard_n$N.log | cut -c1-1500
-BSW_MULTI=deal timeout 400 python scripts/multi_probe.py --max-devices $N > $OUT/${TAG}_multi_probe_deal_n$N.log 2>&1; tail -1 $OUT/${TAG}_multi_probe_deal_n$N.log | cut -c1-1500
 timeout 600 $TR --master-port 29611 bench.py --impl reference --gpus $N --steps 2 --warmup 1 > $OUT/${TAG}_bench_ref_n$N.json 2> $OUT/${TAG}_bench_ref_n$N.err
 tail -c 400 $OUT/${TAG}_bench_ref_n$N.json
 timeout 600 $TR --master-port 29612 bench.py --gpus $N --steps 20 --warmup 3 > $OUT/${TAG}_bench_short8_n$N.json 2> $OUT/${TAG}_bench_short8_n$N.err
 tail -c 1500 $OUT/${TAG}_bench_short8_n$N.json; tail -5 $OUT/${TAG}_bench_short8_n$N.err
-# A/B at N ranks: the direct route's way out (records DMA vs 16-byte results + host pass) where the host fabric bounds e2e
-BSW_DIRECT_OUT=results timeout 300 $TR --master-port 29613 bench.py --gpus $N --steps 10 --warmup 3 --no-split-legs --no-cpu-baseline \
-    > $OUT/${TAG}_bench_short8_n${N}_out_results.json 2> /dev/null
 python - <<PY
 import json
-for tag in ("", "_out_results"):
-    try:
-        d = json.loads(open("$OUT/${TAG}_bench_short8_n$N%s.json" % tag).read().strip().splitlines()[-1])
-        print("e2e drop-in%s: %.1f GCUPS %.2f ms/step; packed %.1f GCUPS" % (tag, d["e2e"]["value"], d["e2e"]["ms_per_step"], d["e2e"]["packed"]["value"]))
-    except Exception as e:
-        print("no line", tag, e)
+try:
+    d = json.loads(open("$OUT/${TAG}_bench_short8_n$N.json").read().strip().splitlines()[-1])
+    print("e2e drop-in: %.1f GCUPS %.2f ms/step; packed %.1f GCUPS" % (d["e2e"]["value"], d["e2e"]["ms_per_step"], d["e2e"]["packed"]["value"]))
+except Exception as e:
+    print("no line", e)
 PY

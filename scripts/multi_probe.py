@@ -1,13 +1,11 @@
 #!/usr/bin/env python
 """ONE engine, ONE call, N devices: strong scaling of the in-call partitioner (contiguous cost-balanced range per
-device, one host thread each) on configs[4]'s divergent pairs and on the large mix, next to the round-robin dealing of
-chunks it replaced (run the script again with BSW_MULTI=deal for that column).
+device, one host thread each) on configs[4]'s divergent pairs and on the large mix.
 
     python scripts/multi_probe.py [--pairs 8000000] [--workload sweep] [--max-devices 8]
 """
 import argparse
 import json
-import os
 import sys
 import time
 from pathlib import Path
@@ -45,8 +43,7 @@ def main():
     pp, pr, pq = gb.pinned_copy(pairs), gb.pinned_copy(ref), gb.pinned_copy(qer)
     batch = gb.PackedBatch.from_pairs(pairs, ref, qer, pinned=True)
     out = gb.pinned_empty(len(pairs), gb.OUTSCORE_DTYPE)
-    mode = os.environ.get("BSW_MULTI", "shard")
-    res = {"workload": args.workload, "pairs": args.pairs, "mode": mode, "points": {}}
+    res = {"workload": args.workload, "pairs": args.pairs, "points": {}}
     base = None
     nd = 1
     while nd <= ngpu:
@@ -67,8 +64,6 @@ def main():
     for nd, p in res["points"].items():
         p["packed_speedup"] = p1["packed_ms"] / p["packed_ms"]
         p["dropin_speedup"] = p1["dropin_ms"] / p["dropin_ms"]
-    (ROOT / "gpurun_out").mkdir(exist_ok=True)
-    (ROOT / "gpurun_out" / f"multi_probe_{args.workload}_{mode}.json").write_text(json.dumps(res, indent=1))
     print(json.dumps(res))
 
 

@@ -1,5 +1,5 @@
 """Pageable (unmodified-driver) route: end-to-end time of bsw_extend on pageable numpy buffers, host pass times, PCIe bytes
-per pair, and the resident kernel time of a batch staged from them.  BSW_STAGED_BYTES=1 = the round-1 byte form of the pass."""
+per pair, and the resident kernel time of a batch staged from them."""
 import os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, genomicsbench_b200 as gb
